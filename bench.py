@@ -5,6 +5,7 @@ depthwise-kernel HBM roofline and the reference's CPU path timed on the same box
   python bench.py [--gpus N --steps K --warmup W]            # this repo's CUDA path
   python bench.py --impl reference [...]                      # the reference's CPU (nn.Conv2d) path
   python -m torch.distributed.run --nproc-per-node N ... bench.py --gpus N ...   (N > 1)
+  python bench.py [...] --dump-outputs DIR                    # also write what the last timed step computed
 
 One JSON line on stdout (rank 0).  A "step" is one fwd+bwd+AdamW pass of the hot path over
 one synthetic batch.  See DESIGN.md "Measurement" for every field.
@@ -62,6 +63,8 @@ def parse():
     p.add_argument("--torch-adamw", action="store_true", help="torch.optim.AdamW(fused=True) instead of slak_b200.optim.FusedAdamW")
     p.add_argument("--watchdog", type=float, default=1500.0, help="abort the process after this many seconds")
     p.add_argument("--no-graph", action="store_true", help="launch every kernel eagerly instead of replaying a CUDA graph")
+    p.add_argument("--dump-outputs", metavar="DIR", default=None,
+                   help="after the timed steps, write what the last one computed to DIR/<name>.npy (see dump_outputs)")
     a = p.parse_args()
     a.cfg = CONFIGS[a.config]
     if a.batch is None:
@@ -345,6 +348,40 @@ def ref_ext_leg(args):
 
 
 # ---------------------------------------------------------------------------------------
+# outputs of the last timed step, for comparing two builds output for output
+# ---------------------------------------------------------------------------------------
+DUMP_SAMPLES = 4 << 20       # parameter / gradient elements kept: 2 x 16 MB of float32, whatever the model's size
+
+
+def dump_outputs(path, loss, logits, params):
+    """What a caller of the training step receives from its last timed step, as float32 .npy files:
+    loss.npy (the loss), logits.npy (the model's output, every micro-step's batch in order), params.npy and grads.npy
+    (the parameters after the optimizer update and the gradients it applied, over the concatenation of
+    net.parameters() in order, at DUMP_SAMPLES positions drawn once from a fixed seed, ascending; all of them when
+    the model has fewer).  The inputs and the initial weights come from fixed seeds, so two runs with the same
+    arguments compute on the same data."""
+    import numpy as np
+    os.makedirs(path, exist_ok=True)
+    sizes = [p.numel() for p in params]
+    total = sum(sizes)
+    if total <= DUMP_SAMPLES:
+        idx = torch.arange(total)
+    else:
+        idx = torch.randperm(total, generator=torch.Generator().manual_seed(0))[:DUMP_SAMPLES].sort().values
+    starts = torch.tensor([0] + sizes).cumsum(0)
+    ps, gs = [], []
+    for i, p in enumerate(params):
+        lo, hi = torch.searchsorted(idx, starts[i : i + 2]).tolist()
+        at = (idx[lo:hi] - starts[i]).to(p.device)
+        ps.append(p.detach().flatten()[at].float())
+        gs.append((p.grad.detach().flatten()[at] if p.grad is not None else torch.zeros(hi - lo, device=p.device)).float())
+    arrays = {"loss": loss.detach().float().reshape(1), "logits": torch.cat([t.detach().float() for t in logits]),
+              "params": torch.cat(ps), "grads": torch.cat(gs)}
+    for name, t in arrays.items():
+        np.save(os.path.join(path, name + ".npy"), t.cpu().numpy())
+
+
+# ---------------------------------------------------------------------------------------
 # this repo's CUDA path
 # ---------------------------------------------------------------------------------------
 def run_ours(args):
@@ -414,12 +451,16 @@ def run_ours(args):
         if not args.torch_adamw:
             opt.attach_masking(mask)                   # p *= mask inside the optimizer launch
 
+    logits = []         # the model's outputs of the latest step (in a captured graph: its static output buffers)
+
     def step_eager():
         # optimizer.zero_grad() as in engine.py:74-86: under graph capture the gradients live in the graph's private pool
         flat.zero_grad()
+        logits.clear()
         for k in range(UF):                              # engine.py:52-80: loss /= update_freq, backward every micro-step
             with torch.autocast("cuda", dtype=torch.bfloat16):
                 out = net(x_dev[k * B:(k + 1) * B])
+                logits.append(out)
                 loss = F.cross_entropy(out.float(), y_dev[k * B:(k + 1) * B])
                 if UF > 1:
                     loss = loss / UF
@@ -445,7 +486,7 @@ def run_ours(args):
     torch.cuda.current_stream().wait_stream(side)
     barrier()
 
-    graph, static_loss, graph_note = None, None, "eager (no CUDA graph)"
+    graph, static_loss, static_logits, graph_note = None, None, None, "eager (no CUDA graph)"
     tagged = []
     use_graph = not args.no_graph
     launches_per_step = None
@@ -457,6 +498,7 @@ def run_ours(args):
             # thread_local: the NCCL watchdog thread's event queries must not invalidate this thread's capture
             with torch.cuda.graph(graph, capture_error_mode="thread_local"):
                 static_loss = step_eager()
+            static_logits = list(logits)
             launches_per_step = ops.launch_count() - l_before
             # the same step once more WITH CUDA events around every kernel group: replayed only outside the timed
             # regions, for the per-kernel roofline table (the ~100 event nodes cost ~0.5 ms per replay)
@@ -484,6 +526,7 @@ def run_ours(args):
         if graph is not None:
             graph.replay()
             out = static_loss
+            logits[:] = static_logits
         else:
             out = step_eager()
         if mask is not None:
@@ -502,11 +545,13 @@ def run_ours(args):
     barrier()
     e0.record()
     for _ in range(args.steps):
-        run_step()
+        last_loss = run_step()
     e1.record()
     barrier()
     clocks = sampler.stop()
     ms = e0.elapsed_time(e1)
+    if args.dump_outputs and rank == 0:     # before the replays below move the weights on
+        dump_outputs(args.dump_outputs, last_loss, logits, params)
     peaks = {}
     try:
         peaks = json.load(open(os.path.join(ROOT, "MEASURED_PEAKS.json")))

@@ -170,8 +170,104 @@ def gen_conv_grid():
     np.savez_compressed(os.path.join(OUT, "ref_conv_grid.npz"), **out)
 
 
+# (N, C, H, W, R, S) of tests/test_oracle.py
+HOST_CASES = [(2, 3, 9, 8, 7, 3), (1, 2, 16, 16, 13, 13), (2, 2, 14, 14, 47, 5), (1, 3, 7, 7, 5, 13), (1, 1, 1, 1, 3, 3)]
+
+
+def gen_ref_host():
+    """The reference's own host-side depthwise convolution (oracle/_ref/libslak_ref.so, built by oracle/Makefile from
+    the reference's CUTLASS headers) on the inputs of tests/test_oracle.py and tests/test_dwconv_gpu.py."""
+    sys.path.insert(0, ROOT)
+    from oracle import dwconv as orc
+    assert orc.ref_available(), "oracle/_ref/libslak_ref.so not built (make -C oracle)"
+    out = {}
+    for case in HOST_CASES:
+        N, C, H, W, R, S = case
+        g = torch.Generator().manual_seed(sum(case) + 1)
+        x = torch.randn(N, C, H, W, generator=g).numpy()
+        dy = torch.randn(N, C, H, W, generator=g).numpy()
+        w = torch.randn(C, 1, R, S, generator=g).numpy()
+        k = "_".join(map(str, case))
+        out[k + ".fwd"] = orc.fwd_ref(x, w)
+        out[k + ".bwd_data"] = orc.bwd_data_ref(dy, w)
+        out[k + ".bwd_filter"] = orc.bwd_filter_ref(dy, x, w.shape)
+    g = torch.Generator().manual_seed(3)                    # integer-valued fills (test_oracle.py)
+    x = torch.randint(-8, 9, (3, 7, 16, 16), generator=g).float()
+    w = torch.randint(-8, 9, (7, 1, 15, 5), generator=g).float()
+    y = orc.fwd_ref(x.numpy(), w.numpy())
+    assert np.array_equal(y, y.astype(np.int16))            # exact integer sums: stored as such
+    out["int.fwd"] = y.astype(np.int16)
+    g = torch.Generator().manual_seed(7)                    # the small GPU case (test_dwconv_gpu.py)
+    x = torch.randn(2, 3, 12, 10, generator=g)
+    torch.randn(2, 3, 12, 10, generator=g)
+    w = torch.randn(3, 1, 7, 5, generator=g)
+    out["small.fwd"] = orc.fwd_ref(x.numpy(), w.numpy())
+    np.savez_compressed(os.path.join(OUT, "ref_host_dwconv.npz"), **out)
+
+
+def gen_dropin():
+    """The reference's models/SLaK.py, sparse_core.py and operator module imported with slak_b200/dropin in place of
+    the CUTLASS example directory (INTEGRATION.md section 1): what they build and call, for
+    tests/test_dropin_reference_cpu.py."""
+    import re
+    sys.path[:0] = [ROOT, os.path.join(ROOT, "slak_b200", "dropin"), REF]
+    shim = types.ModuleType("timm")
+    shim.__path__ = [os.path.join(HERE, "ref_shims", "timm")]
+    sys.modules["timm"] = shim
+    import depthwise_conv2d_implicit_gemm as op
+    import models.SLaK as ref_slak
+    import sparse_core as ref_sparse
+    from slak_b200 import slak
+    assert ref_slak.DepthWiseConv2dImplicitGEMM is op.DepthWiseConv2dImplicitGEMM
+    out = {}
+    ref_slak.use_sync_bn = False
+    slak.use_sync_bn = False
+    net = ref_slak.SLaK_tiny(kernel_size=[51, 49, 47, 13, 5], Decom=True, bn=True, width_factor=0.25)
+    sd = net.state_dict()
+    out["tiny.keys"] = np.array(list(sd.keys()))
+    out["tiny.shapes"] = np.array([",".join(map(str, v.shape)) for v in sd.values()])
+    out["tiny.dtypes"] = np.array([str(v.dtype) for v in sd.values()])
+    out["tiny.dwconv_modules"] = np.array(sum(isinstance(m, op.DepthWiseConv2dImplicitGEMM) for m in net.modules()))
+    torch.Tensor.cuda = lambda self, *a, **k: self
+    opt = torch.optim.SGD(net.parameters(), lr=0.1, momentum=0.9)
+    args = types.SimpleNamespace(device="cpu", fix=False, update_frequency=100, only_L=True, sparse_init="uniform",
+                                 sparsity=0.4, distributed=False)
+    mask = ref_sparse.Masking(opt, train_loader=None, prune_rate_decay=ref_sparse.CosineDecay(0.3, 100), prune_rate=0.3,
+                              prune_mode="magnitude", growth_mode="random", redistribution_mode="none", args=args)
+    mask.add_module(net)
+    out["tiny.mask_names"] = np.array(list(mask.masks.keys()))
+    # the reference's operator module: the native functions it calls and the module it builds
+    ext_py = os.path.join(REF, "cutlass", "examples", "19_large_depthwise_conv2d_torch_extension",
+                          "depthwise_conv2d_implicit_gemm.py")
+    out["op.native_calls"] = np.array(sorted(set(re.findall(r"_extension\.(\w+)\(", open(ext_py).read()))))
+    # kernel merge and BN folding (models/SLaK.py:49-58,102-122) on non-trivial statistics
+    torch.manual_seed(5)
+    for K, small in ((13, 5), (7, 3), (9, None)):
+        kw = dict(in_channels=6, out_channels=6, kernel_size=K, stride=1, groups=6, small_kernel=small,
+                  small_kernel_merged=False, Decom=False, bn=True)
+        ours = slak.ReparamLargeKernelConv(**kw)
+        for b in ours.branches():
+            b.bn.running_mean.normal_(); b.bn.running_var.uniform_(0.5, 2.0)
+            b.bn.weight.data.normal_(1, 0.2); b.bn.bias.data.normal_()
+            b.conv.weight.data.normal_(0, 0.1)
+        theirs = ref_slak.ReparamLargeKernelConv(**kw)
+        theirs.load_state_dict(ours.state_dict())
+        tag = f"merge_{K}_{small}."
+        for k, v in theirs.state_dict().items():
+            out[tag + "sd0." + k] = v.numpy().copy()
+        k2, b2 = theirs.get_equivalent_kernel_bias()
+        out[tag + "kernel"], out[tag + "bias"] = k2.detach().numpy(), b2.detach().numpy()
+        theirs.merge_kernel()
+        for k, v in theirs.state_dict().items():
+            out[tag + "sd1." + k] = v.detach().numpy().copy()
+    np.savez_compressed(os.path.join(OUT, "ref_dropin.npz"), **out)
+
+
 if __name__ == "__main__":
     os.makedirs(OUT, exist_ok=True)
+    if len(sys.argv) > 1 and sys.argv[1] in ("host", "dropin"):   # python oracle/gen_golden.py host | dropin
+        gen_ref_host() if sys.argv[1] == "host" else gen_dropin()
+        sys.exit(0)
     ref_slak, ref_sparse, ref_funcs = import_reference()
     if len(sys.argv) > 1 and sys.argv[1] == "masking":      # python oracle/gen_golden.py masking [tag ...]
         gen_masking(ref_slak, ref_sparse, only=(sys.argv[2:] or None))
